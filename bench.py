@@ -25,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # a run leaves the tree as it found it (it may be read-only)
 
 METRIC = "video-frames/sec + prefill tokens/sec (VideoLLaMA2-7B, 16f@336) at 1/2/4/8 B200"
 FRAMES, PROMPT = 16, 256
@@ -419,7 +420,12 @@ def main():
     ap.add_argument("--no-graphs", action="store_true", help="launch every kernel eagerly instead of replaying CUDA graphs")
     ap.add_argument("--profile-one-step", action="store_true",
                     help="warm up, then run ONE step between cudaProfilerStart/Stop and exit (for `ncu --profile-from-start off`)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (last-position logits, float32) as DIR/<name>.npy, so two "
+                         "builds can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.model == "qwen2_72b" or args.profile_one_step):
+        ap.error("--dump-outputs applies to the timed prefill step of the --impl vl2 single-model workloads")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -492,9 +498,12 @@ def main():
     px_dev = px_host.to(dev)
     mask = torch.ones_like(ids_host, dtype=torch.bool)
 
+    last = {}
+
     def step_resident():
         _, _, _, emb, _ = model.prepare_inputs_labels_for_multimodal(ids_host, mask, None, None, [(px_dev, "video")])
         logits, _ = model.get_model().decoder.prefill(emb[0], all_logits=False)
+        last["logits"] = logits
         return logits
 
     def step_e2e():
@@ -548,6 +557,11 @@ def main():
         sampler.start()
     ms_step, t0, t1 = timed(step_resident, args.steps)
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # copied before anything else runs: with CUDA graphs the logits live in the graph's static output buffer
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "logits.npy"), last["logits"].float().cpu().numpy())
 
     for _ in range(2):
         step_e2e()

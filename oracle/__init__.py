@@ -7,7 +7,8 @@ CPU checkers for the VideoLLaMA2 video->text prefill path:
                    travels to the GPU box; pinned against the real reference by tests/test_oracle_vs_reference.py here
                    and against the committed fixtures in tests/golden/ everywhere.
   * synth.py       configs + deterministic synthetic weights (HF state-dict names) and inputs.
-  * make_golden.py regenerates tests/golden/*.pt from the real reference.
+  * make_golden.py regenerates tests/golden/*.pt from the real reference; make_golden_calls.py records the reference
+                   calls that tests compare with one by one (tests/golden/reference_calls.pt).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this package.
 Parity status: the reference ships no tests or golden vectors for this path (SURVEY.md §4), so the pin is

@@ -1,6 +1,6 @@
 """Exact (integer) parity of the host-side token / splice logic with the reference
-(videollama2/mm_utils.py:277-302, videollama2/model/videollama2_arch.py:161-263) via the committed fixtures, and live
-against the reference functions when /root/reference exists."""
+(videollama2/mm_utils.py:277-302, videollama2/model/videollama2_arch.py:161-263) via the committed fixtures, which
+record what the reference functions returned."""
 import os
 
 import pytest
@@ -63,17 +63,16 @@ def test_splice_plan_edge_cases():
 
 
 def test_live_reference_splice_and_tokenizer():
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("/root/reference not present")
-    import importlib
-    ref_loader.load()
-    ref_mm = importlib.import_module("videollama2.mm_utils")
-    from oracle.make_golden import PROMPTS, ToyTokenizer
+    """Against the reference's tokenizer_multimodal_token as recorded by oracle/make_golden_calls.py, incl. two
+    placeholders and the empty prompt."""
+    from oracle.make_golden import ToyTokenizer
+    from oracle.make_golden_calls import TOKENIZER_PROMPTS
     from videollama2_b200 import mm_utils
+    ref = torch.load(os.path.join(GOLD, "reference_calls.pt"))["tokenizer"]
+    assert [(p, t) for p, t, _ in ref] == TOKENIZER_PROMPTS
     tok = ToyTokenizer()
-    for p, t in PROMPTS + [("a <video> b <video> c", "<video>"), ("", "<video>")]:
-        assert mm_utils.tokenizer_multimodal_token(p, tok, t) == ref_mm.tokenizer_multimodal_token(p, tok, t)
+    for p, t, ref_ids in ref:
+        assert mm_utils.tokenizer_multimodal_token(p, tok, t) == ref_ids
 
 
 def test_keywords_stopping_criteria():
@@ -189,14 +188,13 @@ def test_mm_infer_matches_reference_goldens():
 
 
 def test_mm_infer_matches_live_reference():
-    from oracle import mm_infer_ref, ref_loader
-    if not ref_loader.available():
-        pytest.skip("/root/reference not present: the committed goldens cover this")
-    instruct, modal, mtype, kw = mm_infer_ref.CASES[0]
-    text, call = mm_infer_ref.run_reference(instruct, modal, mtype, torch.zeros((2, 3, 4, 4)), **kw)
+    """The reference's mm_infer on its first case, as recorded by oracle/make_golden_calls.py."""
+    from oracle import mm_infer_ref
+    ref = torch.load(os.path.join(GOLD, "reference_calls.pt"))["mm_infer"]
+    instruct, modal, mtype, kw = mm_infer_ref.CASES[ref["case"]]
     case = {"instruct": instruct, "modal": modal, "model_type": mtype, "kwargs": kw}
     my_text, mine, _ = _my_mm_infer_call(case)
-    assert my_text == text and torch.equal(mine["input_ids"], mm_infer_ref.summarise(call)["input_ids"])
+    assert my_text == ref["text"] and torch.equal(mine["input_ids"], ref["input_ids"])
     import videollama2_b200
     with pytest.raises(ValueError):
         videollama2_b200.mm_infer(None, "x", mm_infer_ref.RecordingModel("videollama2"), mm_infer_ref.ToyChatTokenizer(), modal="audio")
@@ -296,54 +294,19 @@ def test_assemble_state_dict_base_plus_projector(tmp_path):
     assert set(assemble_state_dict(str(path))) == set(llm) | set(proj)
 
 
-class _DecodingToyTokenizer:
-    """Word-piece toy with a decoder: id 3 + i <-> _VOCAB[i]; pieces are concatenated without spaces, so a keyword can
-    straddle several ids (what the decoded-text branch of KeywordsStoppingCriteria exists for)."""
-    bos_token_id = 1
-    _VOCAB = ["he", "llo", " wor", "ld", "hello!", " stop", "x", "y"]
-
-    class _Enc:
-        def __init__(self, ids):
-            self.input_ids = ids
-
-    def __call__(self, text, add_special_tokens=True):
-        ids, rest = [], text
-        while rest:
-            for i, p in sorted(enumerate(self._VOCAB), key=lambda t: -len(t[1])):
-                if rest.startswith(p):
-                    ids.append(3 + i)
-                    rest = rest[len(p):]
-                    break
-            else:
-                raise ValueError(rest)
-        return self._Enc(([self.bos_token_id] if add_special_tokens else []) + ids)
-
-    def batch_decode(self, ids, skip_special_tokens=True):
-        return ["".join(self._VOCAB[int(t) - 3] for t in row if int(t) >= 3) for row in ids]
-
-
 def test_keywords_stopping_criteria_decoded_text_branch_matches_reference():
     """mm_utils.py:332-337: the keyword may be spelled by different ids than tokenizer(keyword) produced; the decoded tail
-    (window = longest keyword, in ids) is searched too.  Compared call by call with the reference class when
-    /root/reference exists."""
+    (window = longest keyword, in ids) is searched too.  Compared call by call with the reference class's answers
+    recorded by oracle/make_golden_calls.py."""
+    from oracle.make_golden_calls import DecodingToyTokenizer, keyword_cases
     from videollama2_b200.mm_utils import KeywordsStoppingCriteria
-    tok = _DecodingToyTokenizer()
+    tok = DecodingToyTokenizer()
     prompt = torch.zeros(1, 2, dtype=torch.long)
     ours = KeywordsStoppingCriteria(["hello"], tok, prompt)
     kw = tok("hello", add_special_tokens=False).input_ids             # ["he", "llo"]
     bang = tok("hello!", add_special_tokens=False).input_ids          # one id spelling "hello!"
     assert len(kw) == 2 and len(bang) == 1
-    x, y = tok("x", add_special_tokens=False).input_ids[0], tok("y", add_special_tokens=False).input_ids[0]
-    cases = [torch.tensor([[x, y] + kw]), torch.tensor([[x, y, x] + bang]), torch.tensor([[x, y, x, y]]),
-             torch.tensor([bang]), torch.tensor([[x] + bang + [y, y, y, y]]), torch.tensor([[x, y, y] + bang + [y]]),
-             torch.tensor([[x, y] + kw, [x, y, y, y]]), torch.tensor([[x] + kw, [y] + kw])]
-    got = [ours(c, None) for c in cases]
+    got = [ours(c, None) for c in keyword_cases(tok)]
     assert got[0] is True and got[2] is False and got[6] is False and got[7] is True
     assert got[1] is True          # id tail differs from tokenizer("hello"), the decoded window contains it
-    from oracle import ref_loader
-    if ref_loader.available():
-        import importlib
-        ref_loader.load()
-        ref_cls = importlib.import_module("videollama2.mm_utils").KeywordsStoppingCriteria
-        ref = ref_cls(["hello"], tok, prompt)
-        assert got == [bool(ref(c, None)) for c in cases]
+    assert got == torch.load(os.path.join(GOLD, "reference_calls.pt"))["keywords_hello"]

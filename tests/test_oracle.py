@@ -1,6 +1,6 @@
 """The CPU oracle (oracle/torch_ref.py) is pinned against (a) the committed golden fixtures produced by the REAL
-reference classes (oracle/make_golden.py) and (b), when /root/reference is present (build container), the reference
-itself run live.  fp32 restatement vs fp32 reference: round-off only (<= 1e-5 relL2)."""
+reference classes (oracle/make_golden.py) and (b) the reference model's own outputs recorded by
+oracle/make_golden_calls.py.  fp32 restatement vs fp32 reference: round-off only (<= 1e-5 relL2)."""
 import os
 
 import pytest
@@ -44,24 +44,21 @@ def test_oracle_bf16_matches_reference_bf16(name):
 
 
 def test_oracle_vs_live_reference():
-    from oracle import ref_loader, synth, torch_ref
-    if not ref_loader.available():
-        pytest.skip("/root/reference not present (GPU box): goldens cover this")
+    """The reference's fp32 model on the tiny config, as recorded in golden/reference_calls.pt
+    (oracle/make_golden_calls.py): logits, the STC connector alone on a batch of two videos, state-dict names/shapes."""
+    from oracle import make_golden_calls, synth, torch_ref
+    ref = torch.load(os.path.join(GOLD, "reference_calls.pt"))
     cfg = synth.CONFIGS["tiny"]
     sd = synth.state_dict(cfg)
     px, ids = synth.inputs(cfg)
-    m = ref_loader.build_reference_model(cfg, torch.float32, sd)
-    with torch.no_grad():
-        res = m(input_ids=ids, attention_mask=torch.ones_like(ids), images=[(px.float(), "video")])
-        stc_in = torch.randn(2, 4, 16, cfg.vision.hidden)
-        stc_ref = m.get_model().mm_projector(stc_in)
+    stc_in = make_golden_calls.stc_input(cfg)
     mine = torch_ref.full_forward(sd, cfg, px, ids, torch.float32)
-    assert rel(mine["logits"], res.logits[0]) < 1e-5
-    assert rel(torch_ref.stc_forward(sd, stc_in, 1, 4, torch.float32), stc_ref) < 1e-5      # batch of 2 videos
+    assert mine["logits"].shape == ref["tiny_logits"].shape and rel(mine["logits"], ref["tiny_logits"]) < 1e-5
+    stc = torch_ref.stc_forward(sd, stc_in, 1, 4, torch.float32)      # batch of 2 videos
+    assert stc.shape == ref["stc_out"].shape and rel(stc, ref["stc_out"]) < 1e-5
     # state-dict contract: names and shapes of the synthetic weights are exactly the reference model's
-    ref_sd = m.state_dict()
     mine_names = {n: tuple(s) for n, s, _ in synth.model_specs(cfg)}
-    assert {k: tuple(v.shape) for k, v in ref_sd.items()} == mine_names
+    assert ref["state_dict_shapes"] == mine_names
 
 
 def test_flop_model_matches_baseline_md():
