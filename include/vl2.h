@@ -8,7 +8,8 @@
  *
  * Conventions
  *  - extern "C", plain pointers + sizes; no torch types.  All data pointers are DEVICE pointers unless named host_*.
- *  - bf16 storage (`uint16_t`-sized), fp32 accumulate.  Row-major, leading dimensions in ELEMENTS.
+ *  - bf16 storage (`uint16_t`-sized), fp32 accumulate.  Row-major, leading dimensions in ELEMENTS.  The one exception is
+ *    vl2_gemv_fp8, whose weights are fp8 E4M3 with a per-row fp32 scale (decode only; prefill weights stay 16-bit).
  *  - `stream` is a cudaStream_t passed as void*.  Calls enqueue work and return; they never synchronise, never
  *    allocate device memory, and are CUDA-graph capturable.
  *  - Every call returns 0 on success or a negative VL2_E_* code; vl2_last_error() gives a thread-local message.
@@ -169,6 +170,13 @@ int vl2_gemm_skinny(const void* A, int a_f32, const void* W, const float* bias, 
  * act as vl2_gemm_skinny.  HBM-bound: 2*N*K bytes. */
 int vl2_gemv_bf16(const void* x, const void* W, const float* bias, const void* residual /* bf16 [N] or NULL */, void* y,
                   int out_f32, int N, int K, int act, float rms_eps, void* stream);
+/* The same GEMV with fp8 weights (opt-in decode weights, `decode_weights="fp8"`): W8 is fp8 E4M3 [N,K] (no NaN codes) and
+ * w_scale fp32 [N] its per-row dequantisation scale, y[N] = act(w_scale[n] * s * W8[n,:] x + bias) (+ residual); with
+ * VL2_ACT_SWIGLU the gate and up rows each carry their own scale.  x, residual and y are the build's 16-bit type.
+ * Requirements: K % 16 == 0, w_scale != NULL, x / W8 16-byte aligned.  HBM-bound: N*K bytes, half of vl2_gemv_bf16's. */
+int vl2_gemv_fp8(const void* x, const void* W8, const float* w_scale, const float* bias,
+                 const void* residual /* bf16 [N] or NULL */, void* y, int out_f32, int N, int K, int act, float rms_eps,
+                 void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Fused attention (FlashAttention-style, tcgen05 QK^T / PV with TMEM accumulators, TMA-staged K/V).

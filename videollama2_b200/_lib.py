@@ -13,7 +13,7 @@ LIB_PATH_F16 = os.environ.get("VL2_LIBVL2_F16") or os.path.join(_HERE, "libvl2_f
 SYMBOLS = [
     "vl2_version", "vl2_storage_dtype", "vl2_last_error", "vl2_launch_count",
     "vl2_gemm_bf16", "vl2_gemm_skinny", "vl2_attention", "vl2_attention_decode", "vl2_debug_attn_trace", "vl2_debug_attn_timeline", "vl2_debug_gemm_trace", "vl2_gemm_plan",
-    "vl2_decode_rope_append", "vl2_attention_decode_dyn", "vl2_gemv_bf16", "vl2_attention_decode_workspace", "vl2_set_pdl", "vl2_l2_prefetch", "vl2_preprocess_frames", "vl2_preprocess_workspace",
+    "vl2_decode_rope_append", "vl2_attention_decode_dyn", "vl2_gemv_bf16", "vl2_gemv_fp8", "vl2_attention_decode_workspace", "vl2_set_pdl", "vl2_l2_prefetch", "vl2_preprocess_frames", "vl2_preprocess_workspace",
     "vl2_layernorm", "vl2_rmsnorm", "vl2_row_sumsq", "vl2_row_stats",
     "vl2_patch_im2col", "vl2_clip_embed_finish",
     "vl2_dwconv3x3_ln_silu", "vl2_se_scale", "vl2_conv3d_im2col",
@@ -116,6 +116,7 @@ def load(dtype=None) -> C.CDLL:
         "vl2_decode_rope_append": [vp, vp, i64, vp, i32, i32, i32, vp, i32, vp],
         "vl2_attention_decode_dyn": [vp, vp, vp, vp, i64, vp, i32, i32, i32, f32, vp, vp],
         "vl2_gemv_bf16": [vp, vp, vp, vp, vp, i32, i32, i32, i32, f32, vp],
+        "vl2_gemv_fp8": [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, f32, vp],
         "vl2_attention_decode_workspace": [i32, i32, i32],
         "vl2_set_pdl": [i32],
         "vl2_l2_prefetch": [vp, C.c_size_t, vp],

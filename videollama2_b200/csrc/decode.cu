@@ -11,22 +11,27 @@ namespace vl2 {
 // Each warp streams its R rows through a private ring of kGemvStages shared-memory stages filled by 1-D bulk copies
 // (cp.async.bulk + mbarrier): the bytes in flight are set by the ring depth, not by how many loads the compiler keeps
 // in registers, so even N = 4096 (one row per warp, 28 warps per SM) keeps > 100 KB per SM outstanding.
+// FP8 = true: W is fp8 E4M3 with one fp32 scale per row (w_scale): y[n] = act(w_scale[n] * s * dot(W8[n,:], x) + ...),
+// N*K bytes.  Same ring, barriers, PDL points and epilogue; a stage then holds 2048 weights and a lane consumes 16 weights
+// (one 16-byte smem read) and 32 bytes of x per step.  Decode weights only: prefill stays on the bf16 GEMM.
 // ---------------------------------------------------------------------------------------------------------
-constexpr int kGemvChunk = 2048;                      // bytes of one row per stage (1024 bf16)
+constexpr int kGemvChunk = 2048;                      // bytes of one row per stage (1024 bf16 or 2048 fp8 weights)
 constexpr int kGemvWarps = 4;
 // Ring depth: R = 1 (N < 8192: o_proj / down_proj / q,k,v) uses 3 stages = 24 KB per CTA so that 7+ CTAs fit on an SM and
 // the 1024-CTA grids of the 4096-row projections run as ONE wave (ncu: with 4 stages 6 CTAs fit -> 1.15 waves, the
-// second one nearly empty); R = 2 uses 4 stages.
-template <int R> struct GemvCfg { static constexpr int kStages = R == 1 ? 3 : 4; };
+// second one nearly empty); R = 2 uses 4 stages.  fp8 always runs R = 2 with 2 stages (32 KB per CTA, 6 CTAs per SM):
+// its rows are half as long, so a CTA's fixed latency (launch, first stage) is spread over half the bytes, and more
+// resident CTAs hide it; 2 x 2 rows x 2 KB per warp in flight still covers a 4096-wide row without a refill.
+template <int R, bool FP8 = false> struct GemvCfg { static constexpr int kStages = FP8 ? 2 : (R == 1 ? 3 : 4); };
 
-template <int R, bool RMS>
+template <int R, bool RMS, bool FP8>
 __global__ void __launch_bounds__(kGemvWarps * 32)
-gemv_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ W, const float* __restrict__ bias,
+gemv_kernel(const __nv_bfloat16* __restrict__ x, const void* __restrict__ W, const float* __restrict__ bias,
             const __nv_bfloat16* __restrict__ residual, void* __restrict__ y, int out_f32, int N, int K, int act,
-            float rms_eps) {
-  constexpr int kGemvStages = GemvCfg<R>::kStages;
+            float rms_eps, const float* __restrict__ w_scale) {
+  constexpr int kGemvStages = GemvCfg<R, FP8>::kStages;
   extern __shared__ __align__(128) uint8_t gemv_smem[];
-  __shared__ uint64_t bars[kGemvWarps][GemvCfg<R>::kStages];
+  __shared__ uint64_t bars[kGemvWarps][GemvCfg<R, FP8>::kStages];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n0 = (blockIdx.x * kGemvWarps + warp) * R;
   if (n0 >= N) return;                                  // whole warp leaves: no block-wide barrier below
@@ -38,11 +43,14 @@ gemv_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict
     fence_barrier_init();
   }
   __syncwarp();
-  const int row_bytes = K * 2;
+  const int row_bytes = FP8 ? K : K * 2;
   const int n_chunks = (row_bytes + kGemvChunk - 1) / kGemvChunk;
   const uint8_t* wrow[R];
 #pragma unroll
-  for (int r = 0; r < R; ++r) wrow[r] = reinterpret_cast<const uint8_t*>(W + (int64_t)min(n0 + r, N - 1) * K);
+  for (int r = 0; r < R; ++r) {
+    if constexpr (FP8) wrow[r] = static_cast<const uint8_t*>(W) + (int64_t)min(n0 + r, N - 1) * K;
+    else wrow[r] = reinterpret_cast<const uint8_t*>(static_cast<const __nv_bfloat16*>(W) + (int64_t)min(n0 + r, N - 1) * K);
+  }
   auto issue = [&](int c) {   // lane 0 only
     const int s = c % kGemvStages;
     const int off = c * kGemvChunk;
@@ -60,45 +68,98 @@ gemv_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict
   float ss = 0.f;
   const uint4* xp = reinterpret_cast<const uint4*>(x);
   const int nk8 = K >> 3;
-  for (int c = 0; c < n_chunks; ++c) {
-    const int s = c % kGemvStages;
-    // refill the stage consumed in the previous iteration (every lane passed the __syncwarp at its end)
-    if (lane == 0 && c + kGemvStages - 1 < n_chunks) issue(c + kGemvStages - 1);
-    uint4 xv[kGemvChunk / 512];
+  if constexpr (FP8) {
+    float acc2[R];    // second chain per row (odd weight pairs): halves the dependent-FMA latency per 16-weight step
 #pragma unroll
-    for (int u = 0; u < kGemvChunk / 512; ++u) {
-      const int idx = c * (kGemvChunk / 16) + u * 32 + lane;
-      xv[u] = idx < nk8 ? __ldg(xp + idx) : make_uint4(0, 0, 0, 0);
-    }
-    mbar_wait(&bar[s], (c / kGemvStages) & 1);
+    for (int r = 0; r < R; ++r) acc2[r] = 0.f;
+    for (int c = 0; c < n_chunks; ++c) {
+      const int s = c % kGemvStages;
+      if (lane == 0 && c + kGemvStages - 1 < n_chunks) issue(c + kGemvStages - 1);
+      uint4 xv[kGemvChunk / 256];   // 16 x values (two uint4) per lane per 512-weight step
 #pragma unroll
-    for (int u = 0; u < kGemvChunk / 512; ++u) {
-      const int idx = c * (kGemvChunk / 16) + u * 32 + lane;
-      if (idx < nk8) {
-        const uint32_t xa[4] = {xv[u].x, xv[u].y, xv[u].z, xv[u].w};
-        float xf[8];
+      for (int u = 0; u < kGemvChunk / 512; ++u) {
+        const int idx = c * (kGemvChunk / 8) + u * 64 + lane * 2;
+        xv[2 * u] = idx < nk8 ? __ldg(xp + idx) : make_uint4(0, 0, 0, 0);
+        xv[2 * u + 1] = idx < nk8 ? __ldg(xp + idx + 1) : make_uint4(0, 0, 0, 0);
+      }
+      mbar_wait(&bar[s], (c / kGemvStages) & 1);
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          xf[2 * j] = bf16_lo(xa[j]);
-          xf[2 * j + 1] = bf16_hi(xa[j]);
-          if (RMS) {
-            ss = fmaf(xf[2 * j], xf[2 * j], ss);
-            ss = fmaf(xf[2 * j + 1], xf[2 * j + 1], ss);
+      for (int u = 0; u < kGemvChunk / 512; ++u) {
+        const int idx = c * (kGemvChunk / 8) + u * 64 + lane * 2;
+        if (idx < nk8) {            // K % 16 == 0: both halves of the 16-weight group are in range
+          const uint32_t xa[8] = {xv[2 * u].x,     xv[2 * u].y,     xv[2 * u].z,     xv[2 * u].w,
+                                  xv[2 * u + 1].x, xv[2 * u + 1].y, xv[2 * u + 1].z, xv[2 * u + 1].w};
+          float xf[16];
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            xf[2 * j] = bf16_lo(xa[j]);
+            xf[2 * j + 1] = bf16_hi(xa[j]);
+            if (RMS) {
+              ss = fmaf(xf[2 * j], xf[2 * j], ss);
+              ss = fmaf(xf[2 * j + 1], xf[2 * j + 1], ss);
+            }
           }
-        }
 #pragma unroll
-        for (int r = 0; r < R; ++r) {
-          const uint4 wq = *reinterpret_cast<const uint4*>(ring + (s * R + r) * kGemvChunk + (u * 32 + lane) * 16);
-          const uint32_t wa[4] = {wq.x, wq.y, wq.z, wq.w};
+          for (int r = 0; r < R; ++r) {
+            const uint4 wq = *reinterpret_cast<const uint4*>(ring + (s * R + r) * kGemvChunk + (u * 32 + lane) * 16);
+            const uint32_t wa[4] = {wq.x, wq.y, wq.z, wq.w};
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            acc[r] = fmaf(xf[2 * j], bf16_lo(wa[j]), acc[r]);
-            acc[r] = fmaf(xf[2 * j + 1], bf16_hi(wa[j]), acc[r]);
+            for (int j = 0; j < 4; ++j) {
+              const float2 w01 = e4m3x2_to_float2(wa[j]);
+              const float2 w23 = e4m3x2_to_float2(wa[j] >> 16);
+              acc[r] = fmaf(xf[4 * j], w01.x, acc[r]);
+              acc[r] = fmaf(xf[4 * j + 1], w01.y, acc[r]);
+              acc2[r] = fmaf(xf[4 * j + 2], w23.x, acc2[r]);
+              acc2[r] = fmaf(xf[4 * j + 3], w23.y, acc2[r]);
+            }
           }
         }
       }
+      __syncwarp();
     }
-    __syncwarp();
+#pragma unroll
+    for (int r = 0; r < R; ++r) acc[r] += acc2[r];
+  } else {
+    for (int c = 0; c < n_chunks; ++c) {
+      const int s = c % kGemvStages;
+      // refill the stage consumed in the previous iteration (every lane passed the __syncwarp at its end)
+      if (lane == 0 && c + kGemvStages - 1 < n_chunks) issue(c + kGemvStages - 1);
+      uint4 xv[kGemvChunk / 512];
+#pragma unroll
+      for (int u = 0; u < kGemvChunk / 512; ++u) {
+        const int idx = c * (kGemvChunk / 16) + u * 32 + lane;
+        xv[u] = idx < nk8 ? __ldg(xp + idx) : make_uint4(0, 0, 0, 0);
+      }
+      mbar_wait(&bar[s], (c / kGemvStages) & 1);
+#pragma unroll
+      for (int u = 0; u < kGemvChunk / 512; ++u) {
+        const int idx = c * (kGemvChunk / 16) + u * 32 + lane;
+        if (idx < nk8) {
+          const uint32_t xa[4] = {xv[u].x, xv[u].y, xv[u].z, xv[u].w};
+          float xf[8];
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            xf[2 * j] = bf16_lo(xa[j]);
+            xf[2 * j + 1] = bf16_hi(xa[j]);
+            if (RMS) {
+              ss = fmaf(xf[2 * j], xf[2 * j], ss);
+              ss = fmaf(xf[2 * j + 1], xf[2 * j + 1], ss);
+            }
+          }
+#pragma unroll
+          for (int r = 0; r < R; ++r) {
+            const uint4 wq = *reinterpret_cast<const uint4*>(ring + (s * R + r) * kGemvChunk + (u * 32 + lane) * 16);
+            const uint32_t wa[4] = {wq.x, wq.y, wq.z, wq.w};
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              acc[r] = fmaf(xf[2 * j], bf16_lo(wa[j]), acc[r]);
+              acc[r] = fmaf(xf[2 * j + 1], bf16_hi(wa[j]), acc[r]);
+            }
+          }
+        }
+      }
+      __syncwarp();
+    }
   }
   // late PDL trigger: the dependent grid is launched while this one drains (its CTAs only prefetch weights until
   // griddepcontrol.wait releases them), never while this grid still has CTAs waiting for an SM slot
@@ -111,7 +172,8 @@ gemv_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict
   float v[R];
 #pragma unroll
   for (int r = 0; r < R; ++r) {
-    v[r] = acc[r] * s;
+    if constexpr (FP8) v[r] = acc[r] * w_scale[min(n0 + r, N - 1)] * s;
+    else v[r] = acc[r] * s;
     if (bias != nullptr && n0 + r < N) v[r] += bias[n0 + r];
   }
   if (act == VL2_ACT_SWIGLU) {   // rows (n0, n0+1) are a (gate, up) pair -> output n0/2      (R == 2)
@@ -348,22 +410,29 @@ using namespace vl2;
 typedef __nv_bfloat16 bf16;
 
 int vl2::launch_gemv(const void* x, const void* W, const float* bias, const void* residual, void* y, int out_f32, int N,
-                       int K, int act, float rms_eps, cudaStream_t stream) {
-  const bool two = act == VL2_ACT_SWIGLU || N >= 8192;
+                       int K, int act, float rms_eps, cudaStream_t stream, const float* w_scale) {
+  const bool fp8 = w_scale != nullptr;
+  const bool two = fp8 || act == VL2_ACT_SWIGLU || N >= 8192;
   const bool rms = rms_eps > 0.f;
   const int rows_per_cta = kGemvWarps * (two ? 2 : 1);
   const int blocks = (N + rows_per_cta - 1) / rows_per_cta;
-  const size_t smem = two ? (size_t)kGemvWarps * GemvCfg<2>::kStages * 2 * kGemvChunk
-                          : (size_t)kGemvWarps * GemvCfg<1>::kStages * kGemvChunk;
-  VL2_SMEM_OPT_IN((gemv_kernel<2, true>), 64 * 1024);
-  VL2_SMEM_OPT_IN((gemv_kernel<2, false>), 64 * 1024);
-#define VL2_GEMV(RR, RMS_)                                                                                                  \
-  launch_kernel(gemv_kernel<RR, RMS_>, dim3(blocks), dim3(kGemvWarps * 32), smem, stream, 1, (const bf16*)x, (const bf16*)W, \
-                bias, (const bf16*)residual, y, out_f32, N, K, act, rms_eps)
-  if (two && rms) VL2_GEMV(2, true);
-  else if (two) VL2_GEMV(2, false);
-  else if (rms) VL2_GEMV(1, true);
-  else VL2_GEMV(1, false);
+  const size_t smem = fp8 ? (size_t)kGemvWarps * GemvCfg<2, true>::kStages * 2 * kGemvChunk
+                     : two ? (size_t)kGemvWarps * GemvCfg<2>::kStages * 2 * kGemvChunk
+                           : (size_t)kGemvWarps * GemvCfg<1>::kStages * kGemvChunk;
+#define VL2_GEMV(RR, RMS_, F8)                                                                                              \
+  launch_kernel(gemv_kernel<RR, RMS_, F8>, dim3(blocks), dim3(kGemvWarps * 32), smem, stream, 1, (const bf16*)x, W, bias,   \
+                (const bf16*)residual, y, out_f32, N, K, act, rms_eps, w_scale)
+  if (fp8) {
+    if (rms) VL2_GEMV(2, true, true);
+    else VL2_GEMV(2, false, true);
+  } else {
+    VL2_SMEM_OPT_IN((gemv_kernel<2, true, false>), 64 * 1024);
+    VL2_SMEM_OPT_IN((gemv_kernel<2, false, false>), 64 * 1024);
+    if (two && rms) VL2_GEMV(2, true, false);
+    else if (two) VL2_GEMV(2, false, false);
+    else if (rms) VL2_GEMV(1, true, false);
+    else VL2_GEMV(1, false, false);
+  }
 #undef VL2_GEMV
   VL2_CHECK_LAUNCH("gemv_kernel");
   return VL2_OK;
@@ -378,6 +447,18 @@ extern "C" int vl2_gemv_bf16(const void* x, const void* W, const float* bias, co
   VL2_REQUIRE(act != VL2_ACT_SWIGLU || (N % 2 == 0 && residual == nullptr), VL2_E_UNSUPPORTED,
               "vl2_gemv_bf16: SWIGLU needs even N and no residual");
   return launch_gemv(x, W, bias, residual, y, out_f32, N, K, act, rms_eps, (cudaStream_t)stream);
+}
+
+extern "C" int vl2_gemv_fp8(const void* x, const void* W8, const float* w_scale, const float* bias, const void* residual,
+                            void* y, int out_f32, int N, int K, int act, float rms_eps, void* stream) {
+  VL2_REQUIRE(N > 0 && K > 0 && K % 16 == 0, VL2_E_BADSHAPE, "vl2_gemv_fp8: need K %% 16 == 0 (N=%d K=%d)", N, K);
+  VL2_REQUIRE(w_scale != nullptr, VL2_E_BADSHAPE, "vl2_gemv_fp8: w_scale (fp32 [N]) is required");
+  VL2_REQUIRE(x && W8 && y && aligned16(x) && aligned16(W8), VL2_E_BADALIGN, "vl2_gemv_fp8: 16-byte alignment");
+  VL2_REQUIRE(act == VL2_ACT_NONE || act == VL2_ACT_SILU || act == 100 || act == VL2_ACT_SWIGLU, VL2_E_UNSUPPORTED,
+              "vl2_gemv_fp8: act %d", act);
+  VL2_REQUIRE(act != VL2_ACT_SWIGLU || (N % 2 == 0 && residual == nullptr), VL2_E_UNSUPPORTED,
+              "vl2_gemv_fp8: SWIGLU needs even N and no residual");
+  return launch_gemv(x, W8, bias, residual, y, out_f32, N, K, act, rms_eps, (cudaStream_t)stream, w_scale);
 }
 
 extern "C" int vl2_l2_prefetch(const void* ptr, size_t bytes, void* stream) {

@@ -507,5 +507,15 @@ __device__ __forceinline__ float bf16_hi(uint32_t u) { return __half2float(__ush
 __device__ __forceinline__ float bf16_lo(uint32_t u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float bf16_hi(uint32_t u) { return __uint_as_float(u & 0xffff0000u); }
 #endif
+// Two fp8 E4M3 codes (low byte = first element) -> fp32, exactly: one cvt to f16x2 (every E4M3 value, subnormals
+// included, is an fp16 value) and two f16 -> f32 conversions.
+__device__ __forceinline__ float2 e4m3x2_to_float2(uint32_t two_codes) {
+  uint32_t h2;
+  asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h2) : "h"((unsigned short)two_codes));
+  float lo, hi;
+  asm("cvt.f32.f16 %0, %1;" : "=f"(lo) : "h"((unsigned short)(h2 & 0xffffu)));
+  asm("cvt.f32.f16 %0, %1;" : "=f"(hi) : "h"((unsigned short)(h2 >> 16)));
+  return make_float2(lo, hi);
+}
 
 }  // namespace vl2

@@ -84,8 +84,9 @@ static inline int grid_for(int64_t work_items, int threads, int max_blocks = 148
   return (int)b;
 }
 
-// M = 1 GEMV launcher (decode.cu); vl2_gemm_skinny routes single-row calls to it.
+// M = 1 GEMV launcher (decode.cu); vl2_gemm_skinny routes single-row calls to it.  w_scale != nullptr: W is fp8 E4M3
+// with one fp32 scale per row (vl2_gemv_fp8).
 int launch_gemv(const void* x, const void* W, const float* bias, const void* residual, void* y, int out_f32, int N, int K,
-                int act, float rms_eps, cudaStream_t stream);
+                int act, float rms_eps, cudaStream_t stream, const float* w_scale = nullptr);
 
 }  // namespace vl2

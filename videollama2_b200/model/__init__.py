@@ -7,6 +7,7 @@ import os
 import torch
 
 from .config import Videollama2Config, VisionConfig
+from .decoder import check_decode_weights
 from .encoder import CLIPVisionTower, SiglipVisionTower, build_vision_tower
 from .projector import STCConnector, STCConnectorV35, build_vision_projector, load_mm_projector
 from .videollama2_mistral import Videollama2MistralConfig, Videollama2MistralForCausalLM
@@ -86,10 +87,12 @@ def assemble_state_dict(model_path: str, model_base=None, config=None):
 
 
 def load_pretrained_model(model_path, model_base=None, model_name=None, load_8bit=False, load_4bit=False,
-                          device_map="auto", device="cuda", use_flash_attn=False, **kwargs):
+                          device_map="auto", device="cuda", use_flash_attn=False, decode_weights="bf16", **kwargs):
     """The reference loader (model/__init__.py:48-193) for LOCAL directories: the SFT-checkpoint branch (:165-180) and the
     base + `mm_projector.bin` branch (:138-164); returns (tokenizer, model, image_processor, context_len).  LoRA / 4-bit /
-    8-bit branches are training artefacts outside the accelerated path."""
+    8-bit branches are training artefacts outside the accelerated path.  `decode_weights="fp8"`: fp8 E4M3 weights for the
+    KV-cache decode steps only (see Videollama2MistralForCausalLM.from_state_dict)."""
+    check_decode_weights(decode_weights)
     if load_8bit or load_4bit:
         raise NotImplementedError("bitsandbytes loading is not supported by the B200 engine")
     if model_name and "lora" in model_name.lower():
@@ -107,7 +110,7 @@ def load_pretrained_model(model_path, model_base=None, model_name=None, load_8bi
     elif tower is not None:
         config.vision_config = VisionConfig.from_dir(tower)     # local directory, or a known hub id (built-in dims)
     sd = assemble_state_dict(model_path, model_base, config)
-    model = VLLMs[model_type].from_state_dict(config, sd, device=device)
+    model = VLLMs[model_type].from_state_dict(config, sd, device=device, decode_weights=decode_weights)
     from transformers import AutoTokenizer
     # the reference loads the SLOW tokenizer for every videollama2 branch (model/__init__.py:146,167): fast and slow
     # Llama / Mistral tokenizers can split differently around special tokens, and tokenizer_multimodal_token tokenizes

@@ -5,7 +5,9 @@ HF:qwen2/modeling_qwen2.py:187-246): RMSNorm -> fused QKV GEMM (+bias for Qwen2)
 -> o_proj(+residual) -> RMSNorm -> gate/up GEMM with SwiGLU epilogue -> down_proj(+residual) -> norm -> lm_head.
 Weights are repacked once: q/k/v concatenated, gate/up rows interleaved so SwiGLU happens inside the GEMM tile, and the
 RMSNorm gains multiplied into the weight columns: the per-layer norms cost no kernel (row statistics are produced by
-the residual GEMM epilogues, the 1/rms factor is applied in the consuming GEMM's epilogue)."""
+the residual GEMM epilogues, the 1/rms factor is applied in the consuming GEMM's epilogue).
+With decode_weights="fp8" the single-token decode streams fp8 E4M3 copies of every linear weight (one fp32 scale per
+output row, vl2_gemv_fp8): half the bytes per token.  Prefill always runs on the 16-bit weights."""
 from __future__ import annotations
 
 import os
@@ -16,9 +18,22 @@ import torch
 from .. import ops
 
 
+DECODE_WEIGHTS = ("bf16", "fp8")
+
+
+def check_decode_weights(decode_weights: str) -> str:
+    if decode_weights not in DECODE_WEIGHTS:
+        raise ValueError(f"decode_weights must be one of {DECODE_WEIGHTS}, not {decode_weights!r}")
+    return decode_weights
+
+
 class DecoderEngine:
-    def __init__(self, config):
+    def __init__(self, config, decode_weights: str = "bf16"):
         self.config = config
+        # "bf16": decode streams the prefill's 16-bit weights; "fp8": E4M3 copies with per-row scales (load_state_dict)
+        self.decode_weights = check_decode_weights(decode_weights)
+        self.layers8: List[Dict[str, torch.Tensor]] = []
+        self.w8: Dict[str, torch.Tensor] = {}
         self.H = config.hidden_size
         self.Hq = config.num_attention_heads
         self.Hkv = config.num_key_value_heads
@@ -58,6 +73,8 @@ class DecoderEngine:
         bf = lambda t: t.to(device=dev, dtype=self.dtype).contiguous()
         f32 = lambda t: t.to(device=dev, dtype=torch.float32).contiguous()
         self.layers = []
+        self.layers8, self.w8 = [], {}
+        fp8 = self.decode_weights == "fp8"
         # RoPE runs in the epilogue of the fused QKV GEMM on ADJACENT column pairs: permute the q / k weight rows (and
         # biases) so that the partners (i, i + D/2) of a head come out as columns (2i, 2i+1).  q.k is invariant under the
         # permutation (same one for q and k), v is untouched, so attention and the KV cache consume the rows as they are.
@@ -75,22 +92,34 @@ class DecoderEngine:
             wqkv = wqkv[qk_perm]          # RoPE partners of every q / k head become adjacent output columns
             wgu = torch.stack([sd[p + "mlp.gate_proj.weight"], sd[p + "mlp.up_proj.weight"]], 1).reshape(
                 2 * self.I, self.H).to(device=dev, dtype=torch.float32)
+            wqkv, wgu = wqkv * g1[None, :], wgu * g2[None, :]
             L = {
-                "wqkv": (wqkv * g1[None, :]).to(self.dtype).contiguous(),
+                "wqkv": wqkv.to(self.dtype).contiguous(),
                 "wo": bf(sd[p + "self_attn.o_proj.weight"]),
-                "wgu": (wgu * g2[None, :]).to(self.dtype).contiguous(),
+                "wgu": wgu.to(self.dtype).contiguous(),
                 "wd": bf(sd[p + "mlp.down_proj.weight"]),
             }
-            del wqkv, wgu
             if p + "self_attn.q_proj.bias" in sd:
                 L["bqkv"] = f32(torch.cat([sd[p + f"self_attn.{n}.bias"] for n in names], 0).to(dev)[qk_perm])
             self.layers.append(L)
+            if fp8:     # quantised from the same fp32 (folded, permuted, interleaved) tensors: one rounding, not two
+                src = {"wqkv": wqkv, "wo": f32(sd[p + "self_attn.o_proj.weight"]), "wgu": wgu,
+                       "wd": f32(sd[p + "mlp.down_proj.weight"])}
+                L8 = {k: v for k, v in L.items() if k.startswith("b")}
+                for k, wf in src.items():
+                    L8[k], L8[k + "_s"] = ops.quantize_fp8_rows(wf)
+                self.layers8.append(L8)
+                del src
+            del wqkv, wgu
+        # final-norm gain folded into the lm_head columns (the GEMV / GEMM epilogue applies 1/rms itself)
+        lm_head = (sd["lm_head.weight"].to(device=dev, dtype=torch.float32)
+                   * sd["model.norm.weight"].to(device=dev, dtype=torch.float32)[None, :])
         self.w = {"embed": bf(sd["model.embed_tokens.weight"]), "norm": bf(sd["model.norm.weight"]),
-                  # final-norm gain folded into the lm_head columns (the GEMV / GEMM epilogue applies 1/rms itself)
-                  "lm_head": (sd["lm_head.weight"].to(device=dev, dtype=torch.float32)
-                                * sd["model.norm.weight"].to(device=dev, dtype=torch.float32)[None, :]
-                                ).to(self.dtype).contiguous(),
+                  "lm_head": lm_head.to(self.dtype).contiguous(),
                   "ones": torch.ones((self.H,), device=dev, dtype=self.dtype)}
+        if fp8:
+            self.w8["lm_head"], self.w8["lm_head_s"] = ops.quantize_fp8_rows(lm_head)
+        del lm_head
         inv = 1.0 / (self.config.rope_theta ** (torch.arange(0, self.D, 2, dtype=torch.int64).float() / self.D))
         self.w["inv_freq"] = inv.to(dev)
         # one table for every position the model can see (8 MB at 32768 x 64): captured graphs keep its address
@@ -162,28 +191,34 @@ class DecoderEngine:
         self._decode_graph = None
 
     # ---- KV-cache decode (one token) -----------------------------------------------------------------------
+    def _decode_set(self):
+        """(per-layer weight dicts, dict holding lm_head) that decode streams.  The fp8 dicts hold every weight `k` as
+        float8_e4m3fn with its per-row scale under `k + "_s"`; the 16-bit dicts have no scales (w_scale=None)."""
+        return (self.layers8, self.w8) if self.decode_weights == "fp8" else (self.layers, self.w)
+
     def decode_step(self, x: torch.Tensor) -> torch.Tensor:
         """x [1,H] bf16 (embedding of the newest token) -> logits fp32 [1,V]; appends K/V at position kv_len.
-        Every linear layer is a weight-streaming GEMV with the RMSNorm in front of it fused (vl2_gemv_bf16), attention
-        is the split-KV vl2_attention_decode."""
+        Every linear layer is a weight-streaming GEMV with the RMSNorm in front of it fused (vl2_gemv_bf16, or
+        vl2_gemv_fp8 with decode_weights="fp8"), attention is the split-KV vl2_attention_decode."""
         if not self.kv:
             raise RuntimeError("decode_step needs prefill(keep_cache=True) first")
         pos = self.kv_len
         if pos >= self.kv[0].shape[0]:
             raise RuntimeError(f"KV cache full ({pos} positions)")
         Hq, Hkv, D = self.Hq, self.Hkv, self.D
-        for i, L in enumerate(self.layers):
+        layers, head = self._decode_set()
+        for i, L in enumerate(layers):
             cache = self.kv[i]
             row = cache[pos:pos + 1]
-            ops.gemv(x, L["wqkv"], bias=L.get("bqkv"), out=row, rms_eps=self.eps)
+            ops.gemv(x, L["wqkv"], w_scale=L.get("wqkv_s"), bias=L.get("bqkv"), out=row, rms_eps=self.eps)
             ops.rope_inplace(row, 1, Hq, Hkv, D, 0, Hq * D, pos, self.w["inv_freq"], interleaved=True)
             o = ops.attention_decode(row[0, : Hq * D], cache[:, Hq * D: (Hq + Hkv) * D], cache[:, (Hq + Hkv) * D:],
                                      n_pos=pos + 1, Hq=Hq, Hkv=Hkv, D=D, scale=D ** -0.5)
-            x = ops.gemv(o, L["wo"], residual=x)
-            h = ops.gemv(x, L["wgu"], act=ops.ACT_SWIGLU, rms_eps=self.eps)
-            x = ops.gemv(h, L["wd"], residual=x)
+            x = ops.gemv(o, L["wo"], w_scale=L.get("wo_s"), residual=x)
+            h = ops.gemv(x, L["wgu"], w_scale=L.get("wgu_s"), act=ops.ACT_SWIGLU, rms_eps=self.eps)
+            x = ops.gemv(h, L["wd"], w_scale=L.get("wd_s"), residual=x)
         self.kv_len = pos + 1
-        return ops.gemv(x, self.w["lm_head"], rms_eps=self.eps, out_dtype=torch.float32)
+        return ops.gemv(x, head["lm_head"], w_scale=head.get("lm_head_s"), rms_eps=self.eps, out_dtype=torch.float32)
 
     # ---- the same step as ONE CUDA graph ---------------------------------------------------------------------
     def _decode_body(self, tok_dev: torch.Tensor, pos_dev: torch.Tensor, stage: torch.Tensor, log=None) -> torch.Tensor:
@@ -192,9 +227,10 @@ class DecoderEngine:
         Hq, Hkv, D = self.Hq, self.Hkv, self.D
         x = torch.index_select(self.w["embed"], 0, tok_dev)
         o = torch.empty((1, Hq * D), device=x.device, dtype=self.dtype)
-        for i, L in enumerate(self.layers):
+        layers, head = self._decode_set()
+        for i, L in enumerate(layers):
             cache = self.kv[i]
-            ops.gemv(x, L["wqkv"], bias=L.get("bqkv"), out=stage, rms_eps=self.eps)
+            ops.gemv(x, L["wqkv"], w_scale=L.get("wqkv_s"), bias=L.get("bqkv"), out=stage, rms_eps=self.eps)
             joined = None
             if self.decode_prefetch_mb > 0:       # fork: weight prefetch into L2 next to the attention phase
                 main = torch.cuda.current_stream()
@@ -205,7 +241,7 @@ class DecoderEngine:
                 self._side_stream.wait_event(fork)
                 with torch.cuda.stream(self._side_stream):
                     budget = int(self.decode_prefetch_mb * 1e6)
-                    n_wo = L["wo"].numel() * 2
+                    n_wo = L["wo"].numel() * L["wo"].element_size()
                     ops.l2_prefetch(L["wo"], min(budget, n_wo))
                     if budget > n_wo:
                         ops.l2_prefetch(L["wgu"], budget - n_wo)
@@ -216,10 +252,10 @@ class DecoderEngine:
                                      pos_dev, Hq=Hq, Hkv=Hkv, D=D, scale=D ** -0.5, out=o)
             if joined is not None:
                 torch.cuda.current_stream().wait_event(joined)
-            x = ops.gemv(o, L["wo"], residual=x)
-            h = ops.gemv(x, L["wgu"], act=ops.ACT_SWIGLU, rms_eps=self.eps)
-            x = ops.gemv(h, L["wd"], residual=x)
-        logits = ops.gemv(x, self.w["lm_head"], rms_eps=self.eps, out_dtype=torch.float32)
+            x = ops.gemv(o, L["wo"], w_scale=L.get("wo_s"), residual=x)
+            h = ops.gemv(x, L["wgu"], w_scale=L.get("wgu_s"), act=ops.ACT_SWIGLU, rms_eps=self.eps)
+            x = ops.gemv(h, L["wd"], w_scale=L.get("wd_s"), residual=x)
+        logits = ops.gemv(x, head["lm_head"], w_scale=head.get("lm_head_s"), rms_eps=self.eps, out_dtype=torch.float32)
         tok_dev.copy_(torch.argmax(logits, dim=1))
         pos_dev.add_(1)
         if log is not None:          # device-side log of the generated ids: the host reads it in chunks, not per token

@@ -10,7 +10,7 @@ import torch
 
 from .. import mm_utils, ops
 from ..constants import IGNORE_INDEX, MODAL_INDEX_MAP, NUM_FRAMES
-from .decoder import DecoderEngine
+from .decoder import DecoderEngine, check_decode_weights
 from .encoder import build_vision_tower
 from .projector import build_vision_projector
 
@@ -18,8 +18,11 @@ from .projector import build_vision_projector
 class Videollama2MetaModel:
     """Holds the tower, the projector and the decoder (reference: Videollama2MetaModel + the HF *Model it is mixed into)."""
 
-    def __init__(self, config, tp_group=None):
+    def __init__(self, config, tp_group=None, decode_weights: str = "bf16"):
         self.config = config
+        check_decode_weights(decode_weights)
+        if tp_group is not None and decode_weights != "bf16":
+            raise NotImplementedError("decode_weights='fp8' is not supported with a tensor-parallel decoder")
         self.vision_tower = None
         self.mm_projector = None
         if getattr(config, "mm_vision_tower", None) is not None:
@@ -29,7 +32,7 @@ class Videollama2MetaModel:
             from .tp_decoder import TPDecoderEngine
             self.decoder = TPDecoderEngine(config, None if tp_group is True else tp_group)
         else:
-            self.decoder = DecoderEngine(config)
+            self.decoder = DecoderEngine(config, decode_weights=decode_weights)
 
     def get_vision_tower(self):
         vision_tower = getattr(self, "vision_tower", None)

@@ -9,6 +9,7 @@ import torch
 
 from .. import ops
 from .config import Videollama2Config
+from .decoder import check_decode_weights
 from .videollama2_arch import Videollama2MetaForCausalLM, Videollama2MetaModel
 
 
@@ -39,23 +40,29 @@ class EngineKVCache:
 class Videollama2MistralForCausalLM(Videollama2MetaForCausalLM):
     config_class = Videollama2MistralConfig
 
-    def __init__(self, config, tp_group=None, **kwargs):
+    def __init__(self, config, tp_group=None, decode_weights: str = "bf16", **kwargs):
         self.config = config
-        self.model = Videollama2MetaModel(config, tp_group=tp_group)
+        self.model = Videollama2MetaModel(config, tp_group=tp_group, decode_weights=decode_weights)
         self.vocab_size = config.vocab_size
         self._device = torch.device("cpu")
 
     # ---- construction -----------------------------------------------------------------------------------------
     @classmethod
-    def from_state_dict(cls, config, state_dict: Dict[str, torch.Tensor], device="cuda", tp_group=None, dtype=None):
+    def from_state_dict(cls, config, state_dict: Dict[str, torch.Tensor], device="cuda", tp_group=None, dtype=None,
+                        decode_weights: str = "bf16"):
         """Build from HF-named weights (the reference's checkpoint format, SURVEY.md §8b) and repack for the kernels.
         `tp_group` (a process group, or True for the default one): shard the decoder tensor-parallel over its ranks
         (model/tp_decoder.py); every rank passes the same full state dict and keeps its slices.
         `dtype`: torch.bfloat16 (default) or torch.float16 - the storage type of weights and activations; float16 runs the
-        fp16 build of the kernel library (libvl2_f16.so), matching the reference's `torch_dtype=float16` loading."""
+        fp16 build of the kernel library (libvl2_f16.so), matching the reference's `torch_dtype=float16` loading.
+        `decode_weights`: "bf16" (default) - KV-cache decode streams the same 16-bit weights as prefill; "fp8" - decode
+        streams fp8 E4M3 copies of every decoder linear weight and lm_head (one fp32 scale per output row, ~1 byte per
+        parameter of extra device memory): about half the bytes per generated token.  Prefill, and so the first new token,
+        is unchanged; later tokens follow the fp8-quantised model.  Not available with `tp_group`."""
+        check_decode_weights(decode_weights)
         if dtype is not None:          # torch.float16 (the reference's inference dtype) or torch.bfloat16
             config.torch_dtype = str(dtype).replace("torch.", "")
-        self = cls(config, tp_group=tp_group)
+        self = cls(config, tp_group=tp_group, decode_weights=decode_weights)
         self.load_state_dict(state_dict, device)
         return self
 

@@ -13,7 +13,7 @@ from ._lib import (ACT_GELU_ERF, ACT_GELU_TANH, ACT_NONE, ACT_QUICK_GELU, ACT_SI
                    check)
 
 __all__ = [
-    "gemm", "gemm_skinny", "attention", "attention_decode", "decode_rope_append", "attention_decode_dyn", "gemv", "decode_workspace", "l2_prefetch", "layernorm", "rmsnorm", "row_sumsq", "row_stats", "patch_im2col", "patch_embed", "clip_embed_finish",
+    "gemm", "gemm_skinny", "attention", "attention_decode", "decode_rope_append", "attention_decode_dyn", "gemv", "quantize_fp8_rows", "decode_workspace", "l2_prefetch", "layernorm", "rmsnorm", "row_sumsq", "row_stats", "patch_im2col", "patch_embed", "clip_embed_finish",
     "dwconv3x3_ln_silu", "se_scale", "conv3d_im2col", "conv3d_k2s2", "rope_inplace", "embed_splice", "launch_count",
     "ACT_NONE", "ACT_QUICK_GELU", "ACT_SILU", "ACT_GELU_ERF", "ACT_GELU_TANH", "ACT_SWIGLU", "ACT_SIGMOID",
 ]
@@ -246,11 +246,18 @@ class pdl:
 
 
 def l2_prefetch(t: torch.Tensor, nbytes: Optional[int] = None) -> None:
-    """Hint the first `nbytes` of a contiguous device tensor into L2 (vl2_l2_prefetch) on the current stream."""
+    """Hint the first `nbytes` of a contiguous device tensor of any dtype (e.g. fp8 decode weights) into L2
+    (vl2_l2_prefetch) on the current stream."""
     _need_cuda(t)
     total = t.numel() * t.element_size()
     n = total if nbytes is None else min(int(nbytes), total)
-    check(_L(t).vl2_l2_prefetch(t.data_ptr(), n, _stream()), "vl2_l2_prefetch")
+    # a byte-level kernel, the same in both builds: a 16-bit tensor uses its own build, any other dtype (fp8 weights) a
+    # build this process already loaded, so that an fp16 model does not load the bf16 library only for this call
+    if t.dtype in _STORAGE:
+        lib = _L(t)
+    else:
+        lib = next(iter(_lib._libs.values())) if _lib._libs else _lib.load()
+    check(lib.vl2_l2_prefetch(t.data_ptr(), n, _stream()), "vl2_l2_prefetch")
 
 
 _decode_ws = {}
@@ -267,25 +274,50 @@ def decode_workspace(device, Hq: int, Hkv: int, D: int) -> torch.Tensor:
     return ws
 
 
+FP8_MAX = 448.0   # largest finite float8_e4m3fn value
+
+
+def quantize_fp8_rows(w: torch.Tensor):
+    """w [N,K] (any float dtype) -> (w8 float8_e4m3fn [N,K], scale fp32 [N]) with w ~= w8 * scale[:, None]: one scale per
+    output row, amax_row / 448 (1 for an all-zero row), round-to-nearest-even after clamping to +-448 so that no NaN
+    code (0x7F / 0xFF) appears.  Load-time weight preparation for the fp8 decode GEMV (vl2_gemv_fp8), in plain torch."""
+    assert w.dim() == 2
+    wf = w.float()
+    amax = wf.abs().amax(dim=1)
+    scale = torch.where(amax > 0, amax / FP8_MAX, torch.ones_like(amax))
+    w8 = (wf / scale[:, None]).clamp_(-FP8_MAX, FP8_MAX).to(torch.float8_e4m3fn)
+    return w8.contiguous(), scale.contiguous()
+
+
 def gemv(x: torch.Tensor, w: torch.Tensor, *, bias: Optional[torch.Tensor] = None, act: int = ACT_NONE,
          residual: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None, rms_eps: float = 0.0,
-         out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
-    """y[1,Nout] = act(s * w[N,K] x + bias) (+ residual); rms_eps > 0 fuses the RMSNorm in front (gain folded into w)."""
-    _need_cuda(x, w, bias, residual, out)
-    _bf16(x, w, residual)
+         out_dtype: Optional[torch.dtype] = None, w_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """y[1,Nout] = act(s * w[N,K] x + bias) (+ residual); rms_eps > 0 fuses the RMSNorm in front (gain folded into w).
+    A float8_e4m3fn `w` (from quantize_fp8_rows) needs its per-row fp32 `w_scale` [N] and runs vl2_gemv_fp8."""
+    fp8 = w.dtype == torch.float8_e4m3fn
+    if fp8 != (w_scale is not None):
+        raise ValueError("gemv: a float8_e4m3fn weight needs w_scale, and only such a weight takes one")
+    _need_cuda(x, w, bias, residual, out, w_scale)
+    _bf16(x, None if fp8 else w, residual)
     assert x.is_contiguous() and w.is_contiguous() and w.dim() == 2 and x.numel() == w.shape[1]
     N, K = w.shape
     if bias is not None:
         assert bias.dtype == torch.float32 and bias.numel() == N
+    if fp8:
+        assert w_scale.dtype == torch.float32 and w_scale.is_contiguous() and w_scale.numel() == N
     n_out = N // 2 if act == ACT_SWIGLU else N
     if out is None:
         out = torch.empty((1, n_out), device=x.device, dtype=out_dtype or x.dtype)
-    assert out.is_contiguous() and out.numel() == n_out and out.dtype in (torch.float32, w.dtype)
+    assert out.is_contiguous() and out.numel() == n_out and out.dtype in (torch.float32, x.dtype)
     if residual is not None:
         assert residual.is_contiguous() and residual.numel() == n_out
-    check(_L(w).vl2_gemv_bf16(x.data_ptr(), w.data_ptr(), _ptr(bias), _ptr(residual), out.data_ptr(),
-                                    1 if out.dtype == torch.float32 else 0, N, K, act, float(rms_eps), _stream()),
-          "vl2_gemv_bf16")
+    out_f32 = 1 if out.dtype == torch.float32 else 0
+    if fp8:
+        check(_L(x).vl2_gemv_fp8(x.data_ptr(), w.data_ptr(), w_scale.data_ptr(), _ptr(bias), _ptr(residual),
+                                 out.data_ptr(), out_f32, N, K, act, float(rms_eps), _stream()), "vl2_gemv_fp8")
+    else:
+        check(_L(w).vl2_gemv_bf16(x.data_ptr(), w.data_ptr(), _ptr(bias), _ptr(residual), out.data_ptr(),
+                                  out_f32, N, K, act, float(rms_eps), _stream()), "vl2_gemv_bf16")
     return out
 
 
